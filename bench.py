@@ -6,6 +6,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the CPU restatement of the reference, same metric
     python bench.py --workload sweep          # BASELINE configs[4]: N in {1k,5k,20k,100k} on the conv4_3 shape
+    python bench.py ... --dump-outputs DIR    # also writes the results of the last timed step as DIR/*.npy
 
 One "step" = the whole hot path (sparse-point im2col -> Gram statistics -> LASSO channel
 selection -> least-squares reconstruction) over one pool of layer problems.
@@ -69,7 +70,15 @@ def parse():
     ap.add_argument("--workload", default="vgg16", choices=["vgg16", "resnet50", "sweep"],
                     help="vgg16 = BASELINE configs[1] (13 conv layers); resnet50 = configs[3] (48 bottleneck problems); "
                          "sweep = configs[4] (Gram roofline and LASSO data-form kernel against N)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (see dump_outputs); "
+                         "the inputs are seeded, so two builds run with the same arguments can be compared file by file")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "cpb200" or args.workload == "sweep"):
+        ap.error("--dump-outputs needs the GPU arm of the vgg16 or resnet50 workload")
+    return args
 
 
 def config_dict(args, base, world):
@@ -379,6 +388,31 @@ def parity_check(shapes, datas, results, names):
     return out
 
 
+DUMP_W_BYTES = 56 << 20  # all W files together; masks, biases and the two scalar arrays take well under 8 MB more
+
+
+def dump_outputs(out_dir, indices, shapes, results):
+    """Writes the results of one step of the pool (problem i of the pool is prefixed %03d): <i>_<layer>_mask (kept input
+    channels, float32 0/1), <i>_<layer>_W and <i>_<layer>_b (reconstructed weights and bias, float64), and alpha /
+    nprobe (the accepted alpha and the number of probes of every problem, in pool order).  A layer whose W could exceed
+    its share of DUMP_W_BYTES is sampled by output channel: the rows are a fixed seeded draw that depends only on the
+    layer's shape, never on the outputs, so two builds store the same rows."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_W_BYTES // 8 // len(results)  # fp64 values of W per problem
+    for i, s, r in zip(indices, shapes, results):
+        name = os.path.join(out_dir, "%03d_%s_" % (i, s.name))
+        W = r.W.cpu().numpy().reshape(s.n, -1)
+        if s.n * s.K > cap:  # s.K columns if every input channel were kept
+            W = W[np.sort(np.random.RandomState(i).choice(s.n, max(1, cap // s.K), replace=False))]
+        np.save(name + "mask.npy", np.asarray(r.idxs, dtype=np.float32))
+        np.save(name + "W.npy", W.astype(np.float64))
+        np.save(name + "b.npy", r.b.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "alpha.npy"), np.array([r.alpha for r in results], dtype=np.float64))
+    np.save(os.path.join(out_dir, "nprobe.npy"), np.array([r.nprobe for r in results], dtype=np.float64))
+
+
 # ------------------------------------------------------------------------------ GPU arm
 def run_gpu(args):
     import numpy as np
@@ -479,6 +513,8 @@ def run_gpu(args):
         sampler.start()
     ms, launches, res, host_issue, _ = timed(args.steps, lambda: step(False))
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:  # before any later leg reuses the engine's buffers
+        dump_outputs(args.dump_outputs, mine, my_shapes, res)
     total_layers = len(shapes) * args.steps
     value = total_layers / (ms / 1e3)
 

@@ -240,7 +240,7 @@ def run_r3_cases(NET, CF, D):
             out["feats__" + nm] = feats_dict[nm]
         out["alpha_final"] = CF.alpha
         out["rng_after"] = np.random.randint(0, 1 << 30)
-        np.savez_compressed(os.path.join(OUT, "%s.npz" % name), **out)
+        np.savez_compressed(os.path.join(OUT, "%s.npz" % name), **cases.compact_r3_golden(out, spec))
         print(name, "WPQ keys", sorted(str(k) for k in WPQ), "kept", {k: int(v.sum()) for k, v in net.selection.items()},
               "alpha", CF.alpha)
 

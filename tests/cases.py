@@ -1,6 +1,9 @@
 """Seeded input generators shared by oracle/make_golden.py (which runs the real reference on
 them) and the tests (which regenerate the same inputs and compare against the stored
 reference outputs).  numpy's legacy RandomState stream is stable across versions."""
+import hashlib
+import os
+
 import numpy as np
 
 
@@ -168,3 +171,52 @@ R3_CASES = {
     "r3_small": dict(gen=dict(B=4, H=12, widths=(12, 28, 56, 96), nimgbatches=20, seed=61), nBatches=20, P=10,
                      np_seed=71),
 }
+
+
+def digest(a):
+    """sha256 of an array's shape and values (as float64, -0.0 taken as 0.0): equal digests <=> equal arrays, the
+    condition np.testing.assert_array_equal checks."""
+    a = np.ascontiguousarray(a, dtype=np.float64) + 0.0
+    h = hashlib.sha256(repr(a.shape).encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
+
+
+def _r3_first_snapshot(spec):
+    """The live weights / biases the R3 walk starts from: the case's seeded inputs."""
+    _, _, weights, biases = r3_inputs(**spec["gen"])
+    return {"snap__0__%s__%s" % (kind, nm): v[nm] for kind, v in (("w", weights), ("b", biases)) for nm in v}
+
+
+def _r3_expand(stored, spec):
+    g = dict(stored)
+    for k, v in _r3_first_snapshot(spec).items():
+        assert digest(v) == str(g.pop("sha256__" + k)), "the seeded inputs no longer reproduce the golden's " + k
+        g[k] = v
+    for i in range(len(g["snap_stages"])):  # the final state of a layer is its latest snapshot
+        for k in [k for k in g if k.startswith("snap__%d__" % i)]:
+            kind, nm = k.split("__")[2:]
+            g["%s__%s" % (kind, nm)] = g[k]
+    return g
+
+
+def compact_r3_golden(full, spec):
+    """What the golden file of an R3 case stores of the full record (oracle/make_golden.py: run_r3_cases), to stay small:
+    the sampled features and the first snapshot (the seeded inputs) as digests, and no final w__ / b__ (the latest
+    snapshot of each layer).  load_r3_golden rebuilds the record; the features stay digests (sha256__feats__<layer>),
+    compared with digest()."""
+    out = {}
+    for k, v in full.items():
+        if k.startswith(("feats__", "snap__0__")):
+            out["sha256__" + k] = digest(v)
+        elif not k.startswith(("w__", "b__")):
+            out[k] = v
+    back = _r3_expand(out, spec)
+    assert all(np.array_equal(back[k], v) for k, v in full.items() if not k.startswith("feats__")), "lossy"
+    return out
+
+
+def load_r3_golden(golden_dir, name):
+    """The reference's R3 record of R3_CASES[name] as a dict (see compact_r3_golden)."""
+    with np.load(os.path.join(golden_dir, "%s.npz" % name)) as z:
+        return _r3_expand({k: z[k] for k in z.files}, R3_CASES[name])

@@ -1,7 +1,6 @@
 """GPU: Net.R3 -- the reference's whole 3C walk (spatial decomposition, channel decomposition, channel pruning, each
 stage re-extracting features through the weights the previous ones rewrote) -- against the golden written by the
 reference's OWN Net.R3 (oracle/make_golden.py: run_r3_cases), plus the frozen-points pickle round trip."""
-import os
 import pickle
 
 import numpy as np
@@ -60,7 +59,7 @@ def _frozen_net(engine, golden_dir, name, mode):
     from cpb200.lib import cfgs
 
     spec = cases.R3_CASES[name]
-    g = np.load(os.path.join(golden_dir, "%s.npz" % name))
+    g = cases.load_r3_golden(golden_dir, name)
     engine.gram_mode = mode
     net, images = build_net(engine, spec, NumpyConvForward)
     cfgs.c.nBatches, cfgs.c.nPointsPerLayer = spec["nBatches"], spec["P"]
@@ -69,7 +68,7 @@ def _frozen_net(engine, golden_dir, name, mode):
     np.random.seed(spec["np_seed"])
     feats_dict, points_dict = net.freeze()
     for nm in net.convs:
-        np.testing.assert_array_equal(feats_dict[nm], g["feats__" + nm])  # same points, same features
+        assert cases.digest(feats_dict[nm]) == g["sha256__feats__" + nm], nm  # same points, same features
     assert points_dict["data"] == tuple(images[0].shape) and (0, 0) in points_dict and (0, 1) in points_dict
     return spec, g, net, images
 
@@ -119,7 +118,7 @@ def test_r3_free_running_walk(engine, golden_dir, name, mode):
     WPQ, new_pt = net.R3()
     assert cfgs.alpha == float(g["alpha_final"])
     assert np.random.randint(0, 1 << 30) == int(g["rng_after"])
-    for k in [k for k in g.files if k.startswith("sel__")]:
+    for k in [k for k in g if k.startswith("sel__")]:
         assert np.array_equal(net.selection[k[5:]], g[k]), k
     _, specs, _, _ = cases.r3_inputs(**spec["gen"])
 
@@ -134,10 +133,10 @@ def test_r3_free_running_walk(engine, golden_dir, name, mode):
         return x
 
     live = forward({k: v.cpu().numpy() for k, v in net._w.items()}, {k: v.cpu().numpy() for k, v in net._b.items()})
-    ref = forward({k[3:]: g[k] for k in g.files if k.startswith("w__")}, {k[3:]: g[k] for k in g.files if k.startswith("b__")})
+    ref = forward({k[3:]: g[k] for k in g if k.startswith("w__")}, {k[3:]: g[k] for k in g if k.startswith("b__")})
     e_out = float(np.linalg.norm(live - ref) / np.linalg.norm(ref))
     worst = 0.0
-    for k in [k for k in g.files if k.startswith("w__")]:
+    for k in [k for k in g if k.startswith("w__")]:
         worst = max(worst, float(np.linalg.norm(net._w[k[3:]].cpu().numpy() - g[k]) / np.linalg.norm(g[k])))
     print("R3 %s mode %d free running: network output deviates %.2e, worst weight tensor %.2e" % (name, mode, e_out, worst))
     assert e_out <= (1e-3 if mode == 0 else 2e-2) and worst <= (1e-3 if mode == 0 else 5e-2)

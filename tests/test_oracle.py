@@ -223,7 +223,7 @@ class StageSync:
         stages = [str(x) for x in self.g["snap_stages"]]
         assert self.i < len(stages) and stage == stages[self.i], (self.i, stage, stages)
         pre = "snap__%d__" % self.i
-        for key in [k for k in self.g.files if k.startswith(pre)]:
+        for key in [k for k in self.g if k.startswith(pre)]:
             kind, nm = key[len(pre):].split("__")
             ref = self.g[key]
             live = np.asarray(self.get(kind, nm), dtype=np.float64)
@@ -245,16 +245,16 @@ class StageSync:
 def r3_compare(golden, WPQ, selection, weights, biases, tol_inv=1e-6, tol_fac=1e-5):
     """Compares an R3 outcome with the reference's golden: selections exactly; sign-invariant quantities (live
     weights/biases, the P-layer biases) tightly; the individual V / H / P factors up to the sign of each component."""
-    for k in [k for k in golden.files if k.startswith("sel__")]:
+    for k in [k for k in golden if k.startswith("sel__")]:
         assert np.array_equal(selection[k[5:]], golden[k]), k
     worst = 0.0
-    for k in [k for k in golden.files if k.startswith("w__")]:
+    for k in [k for k in golden if k.startswith("w__")]:
         nm = k[3:]
         e = np.linalg.norm(weights[nm] - golden[k]) / np.linalg.norm(golden[k])
         eb = np.abs(biases[nm] - golden["b__" + nm]).max() / max(1.0, np.abs(golden["b__" + nm]).max())
         worst = max(worst, e, eb)
         assert e <= tol_inv and eb <= tol_inv, (nm, e, eb)
-    for k in [k for k in golden.files if k.startswith("WPQ__")]:
+    for k in [k for k in golden if k.startswith("WPQ__")]:
         parts = k[5:].split("__")
         key = (parts[0], int(parts[1])) if len(parts) == 2 else parts[0]
         got, ref = np.asarray(WPQ[key]), golden[k]
@@ -279,7 +279,7 @@ def r3_compare(golden, WPQ, selection, weights, biases, tol_inv=1e-6, tol_fac=1e
 @pytest.mark.parametrize("name", list(cases.R3_CASES))
 def test_r3_walk_matches_reference_golden(golden_dir, name):
     spec = cases.R3_CASES[name]
-    g = np.load(os.path.join(golden_dir, "%s.npz" % name))
+    g = cases.load_r3_golden(golden_dir, name)
     images, specs, weights, biases = cases.r3_inputs(**spec["gen"])
     net = O.NumpyNet(specs, weights, biases)
     np.random.seed(spec["np_seed"])
@@ -290,7 +290,7 @@ def test_r3_walk_matches_reference_golden(golden_dir, name):
     for b in range(spec["nBatches"]):
         pd[(b, 0)] = images[b % len(images)]
     for nm in net.convs:
-        np.testing.assert_array_equal(feats[nm], g["feats__" + nm])
+        assert cases.digest(feats[nm]) == g["sha256__feats__" + nm], nm
     net._feats_dict, net._points_dict = feats, pd
     st = O.DictState(alpha=1e-3)
     sync = StageSync(g, lambda kind, nm: (net.weights if kind == "w" else net.biases)[nm], None, tol=1e-6)
